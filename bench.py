@@ -16,6 +16,7 @@ oracle's run of the same workload (made once, outside the timed regions, on host
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
            --master-port 29500 bench.py --gpus 8 --steps 5 --warmup 3
     python bench.py --impl reference          # the CPU oracle (port of the reference path) on the host cores
+    python bench.py --dump-outputs out/       # also write what the last timed step computed to out/*.npy (see dump_outputs)
 """
 import argparse
 import json
@@ -191,6 +192,45 @@ def time_oracle(args, nodes, repeats=3):
                       f"one pinned worker per physical core", "seconds": r["seconds"], "ticks": r["ticks"]}
 
 
+DUMP_BYTES = 64 << 20                                    # --dump-outputs: all files together stay below this
+DUMP_SEED = 20240601                                     # fixed: the same node ids are sampled on every run
+
+
+def dump_outputs(outdir, sc, g, read_back, ticks, ok, gather):
+    """Write what the last timed step computed, as a caller of the path receives it, to outdir/<name>.npy (float64: every value is
+    an integer below 2**53).  Per-node vectors come from the end-to-end read-back and are sampled at the same node ids on every run:
+      node_ids                      the sampled node ids (ascending)
+      member_status_slot<s>         MemberStatus of tracked subject s in each sampled node's view
+      status_ltime_slot<s>          its status Lamport time
+      lamport_time                  each sampled node's Lamport clock
+      convergence                   [tick of quiescence, 1 if converged]
+      stats                         serfsim_stats_t in field order (Stats._fields_)
+      state_hash                    [high 32 bits, low 32 bits] of the final state hash
+    Every rank takes part (stats, state hash and the gather are collective); rank 0 writes."""
+    from serf_b200 import Stats
+    per_node = 2 + 2 * sc.slots                          # node id, clock, status and status time per slot
+    k = min(sc.n, 1 << 20, (DUMP_BYTES - (1 << 16)) // (8 * per_node))
+    ids = np.sort(np.random.default_rng(DUMP_SEED).choice(sc.n, size=k, replace=False))
+    mine = ids[(ids >= g.first) & (ids < g.first + g.count)]
+    at = mine - g.first
+    local = {"node_ids": mine, "lamport_time": read_back["clock"].numpy().view(np.uint32)[at]}
+    for s in range(sc.slots):
+        local[f"member_status_slot{s}"] = read_back["status"][s].numpy()[at]
+        local[f"status_ltime_slot{s}"] = read_back["ltime"][s].numpy().view(np.uint32)[at]
+    st, h = g.stats(), int(g.state_hash())
+    parts = gather(local)
+    if parts is None:
+        return
+    out = {name: np.concatenate([p[name] for p in parts]) for name in local}
+    assert (out["node_ids"] == ids).all()
+    out["convergence"] = np.array([ticks, int(ok)])
+    out["stats"] = np.array([st[name] for name, _ in Stats._fields_])
+    out["state_hash"] = np.array([h >> 32, h & 0xFFFFFFFF])
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(outdir, name + ".npy"), a.astype(np.float64))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -232,7 +272,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="A/B: leave the driver thread where the OS scheduler puts it")
     ap.add_argument("--no-check", action="store_true", help="skip the full-size oracle run every step is checked against")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                                                          "(a fixed sample of the per-node results, at most 64 MB; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -346,7 +392,7 @@ def main():
     t0 = time.perf_counter()
     d2h = 0
     for k in range(args.steps):
-        _, _, _, _, ob = one_step(pins[k & 1])
+        last_ticks, last_ok, _, _, ob = one_step(pins[k & 1])
         d2h = ob
     g.results_wait()                                     # the last copies have landed in host memory
     sync_all()
@@ -361,6 +407,14 @@ def main():
         others = np.delete(stv, subj - lo) if lo <= subj < hi else stv
         if int((others != MemberStatus.LEFT).sum()) > 8:
             raise SystemExit("bench self-check FAILED: the status vector read back end to end is not the converged one")
+    if args.dump_outputs:                                # the last end-to-end step: its read-back is what a caller receives
+        def gather(local):
+            if world == 1:
+                return [local]
+            parts = [None] * world
+            dist.all_gather_object(parts, local)
+            return parts if rank == 0 else None
+        dump_outputs(args.dump_outputs, sc, g, pins[(args.steps - 1) & 1], last_ticks, last_ok, gather)
 
     t = torch.tensor([dev_ms, wall_e2e, wall_dev], dtype=torch.float64, device="cuda")
     if world > 1:
