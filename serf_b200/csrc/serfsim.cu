@@ -138,8 +138,6 @@ struct serfsim {
   int grid_sv = 0;                 // grid of the single-view kernel
   u32 tick = 0;
   bool has_topo = false;
-  u32 stage_col_bytes = 0;         // 0: direct-load kernel; else bytes of CSR per TMA stage
-  u32 max_tile_edges = 0;          // largest 16-byte-aligned CSR span of one 256-node tile (sizes the TMA stage)
   u32 ahead = 1;                   // multi-slot tick kernel: software pipelining of saturated ticks (SERFSIM_AHEAD=0 / 1 / 2, tick_kernel.cuh)
   u32 udeg = 0;                    // uniform out-degree of the shard's rows (0: degrees differ)
   std::vector<serfsim_tick_row_t> rows;   // rows pulled from the device so far (global sums when sharded)
@@ -176,8 +174,6 @@ struct serfsim {
   serfsim_barrier_fn barrier = nullptr; serfsim_allreduce_u64_fn allreduce = nullptr; void* comm_user = nullptr;
   std::vector<void*> ipc_opened;
   bool tick_timing = false;
-  size_t l2_persist_max = 0, l2_window_max = 0;
-  bool l2_window = false;           // SERFSIM_L2_WINDOW=1: stream access-policy window over the inbox being written
   bool no_skip = false;             // SERFSIM_NO_SKIP=1: process every tile every tick (A/B measurements)
   bool compact = true;              // SERFSIM_COMPACT=0: tile-by-tile walk in unsaturated ticks too (A/B measurements)
   // asynchronous result read-back (serfsim_results_async): extraction into a ring of staging buffers on the launch stream,
@@ -285,7 +281,6 @@ int launch_ticks(serfsim* h, u32 n) {
     p.kinds_cur = h->d_kinds + ((size_t)t + 1) * 4;
     p.overflow = h->d_overflow;
     p.hot_rd = h->d_hot[(t & 1) ^ 1]; p.hot_wr = h->d_hot[t & 1];
-    p.stage_col_bytes = h->stage_col_bytes;
     p.reap_now = (h->cfg.reap_interval_ticks && ((t + 1) % h->cfg.reap_interval_ticks) == 0) ? 1u : 0u;
     p.tombstone_ticks = h->cfg.tombstone_timeout_ticks; p.reconnect_ticks = h->cfg.reconnect_timeout_ticks; p.intent_ticks = h->cfg.recent_intent_timeout_ticks;
     p.stride = h->stride; p.n_tiles = h->n_tiles; p.tiles_per_cta = (h->n_tiles + h->grid - 1) / h->grid;
@@ -313,16 +308,6 @@ int launch_ticks(serfsim* h, u32 n) {
     if (h->tick_timing) {
       while (h->tick_ev.size() < 2 * ((size_t)t + 1)) { cudaEvent_t e; CU(cudaEventCreate(&e)); h->tick_ev.push_back(e); }
       CU(cudaEventRecord(h->tick_ev[2 * (size_t)t], h->stream));
-    }
-    if (h->l2_window && h->l2_window_max) {
-      cudaStreamAttrValue av{};
-      const size_t bytes = (size_t)3 * h->R * h->stride * sizeof(u32);
-      av.accessPolicyWindow.base_ptr = h->d_inbox[t & 1];
-      av.accessPolicyWindow.num_bytes = std::min(bytes, h->l2_window_max);
-      av.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)h->l2_persist_max / (double)std::max<size_t>(1, av.accessPolicyWindow.num_bytes));
-      av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-      av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-      CU(cudaStreamSetAttribute(h->stream, cudaStreamAttributeAccessPolicyWindow, &av));
     }
     if (h->ue_table.n) {                       // user-event tick: needs the pre-operation up flags and op bits, so it runs first
       UeParams u{};
@@ -718,24 +703,9 @@ int serfsim_create(const serfsim_config_t* cfg, serfsim_t** out) {
   const u32 ones[4] = {0x40000000u, 0x40000000u, 0x40000000u, 1u};   // multi-GPU: every inbox plane may hold entries, every tick is dense
   CUB(cudaMemcpy(h->d_ones, ones, 16, cudaMemcpyHostToDevice));
   CUB(cudaMemcpy(h->d_subj, h->subj.data(), h->R * 4, cudaMemcpyHostToDevice));
-  {
-    const char* e = getenv("SERFSIM_MINB");
-    h->ctas_per_sm = (h->R == 1) ? ((e && atoi(e) == 5) ? 5 : (cfg->world_size > 1 ? tick_ctas_per_sm_r1s() : tick_ctas_per_sm_r1())) : tick_ctas_per_sm_rn();
-  }
+  h->ctas_per_sm = (h->R == 1) ? (cfg->world_size > 1 ? tick_ctas_per_sm_r1s() : tick_ctas_per_sm_r1()) : tick_ctas_per_sm_rn();
   h->grid = tick_grid_size(h->count, h->ctas_per_sm);
   h->grid_sv = tick_grid_size(h->count, cfg->world_size > 1 ? tick_ctas_per_sm_r1s() : tick_ctas_per_sm_r1());
-  {
-    // L2 set-aside for persisting (evict_last) lines: the randomly addressed inbox planes live there
-    int max_persist = 0, max_window = 0;
-    cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-    cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-    h->l2_persist_max = (size_t)max_persist; h->l2_window_max = (size_t)max_window;
-    int want = 0;        // measured: a 79 MB persisting carve-out makes the plateau tick 35 % slower (profiles/r1_notes.md)
-    if (const char* e = getenv("SERFSIM_L2_PERSIST")) want = atoi(e);
-    if (want && max_persist > 0) cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist);
-    if (const char* e = getenv("SERFSIM_L2_WINDOW")) h->l2_window = atoi(e) != 0;
-    if (getenv("SERFSIM_VERBOSE")) fprintf(stderr, "serfsim: L2 persisting max %d B, window max %d B, persist %d window %d\n", max_persist, max_window, want, (int)h->l2_window);
-  }
   if (const char* e = getenv("SERFSIM_NO_SKIP")) h->no_skip = atoi(e) != 0;
   if (const char* e = getenv("SERFSIM_COMPACT")) h->compact = atoi(e) != 0;
   if (const char* e = getenv("SERFSIM_AHEAD")) h->ahead = (u32)std::min(2, std::max(0, atoi(e)));
@@ -814,13 +784,7 @@ int serfsim_set_topology_csr(serfsim_t* h, const uint64_t* row_ptr, const uint32
   const u64 ne = e1 - e0;
   h->udeg = (h->count && ne % h->count == 0) ? (u32)(ne / h->count) : 0u;
   for (u32 i = 0; i <= h->count && h->udeg; ++i) if (rp[i] != (u64)i * h->udeg) h->udeg = 0;
-  if (const char* e = getenv("SERFSIM_UDEG")) { if (!atoi(e)) h->udeg = 0; }   // A/B: force the general path
   for (size_t i = h->count + 1; i < rp.size(); ++i) rp[i] = (u32)ne;      // padding rows: degree 0
-  h->max_tile_edges = 0;
-  for (u32 b = 0; b < h->count; b += 256) {
-    const u32 lo = rp[b] & ~3u, hi = (rp[std::min<u32>(b + 256, h->count)] + 3u) & ~3u;
-    h->max_tile_edges = std::max(h->max_tile_edges, hi - lo);
-  }
   for (u64 i = 0; i < ne; ++i) if (col_idx[e0 + i] >= h->N) return fail(SERFSIM_E_INVAL, "col_idx out of range");
   cudaFree(h->d_rowptr); cudaFree(h->d_col); h->d_rowptr = nullptr; h->d_col = nullptr;
   CU(cudaMalloc(&h->d_rowptr, rp.size() * 4));
@@ -828,16 +792,7 @@ int serfsim_set_topology_csr(serfsim_t* h, const uint64_t* row_ptr, const uint32
   CU(cudaMemset(h->d_col, 0, (ne + 8) * 4));
   CU(cudaMemcpy(h->d_rowptr, rp.data(), rp.size() * 4, cudaMemcpyHostToDevice));
   if (ne) CU(cudaMemcpy(h->d_col, col_idx + e0, ne * 4, cudaMemcpyHostToDevice));
-  // TMA pipeline (single-slot runs): a stage holds the largest tile's CSR span if that is at most 48 KB
-  h->stage_col_bytes = 0;
-  {
-    int use = 0;   // measured (profiles/): the direct-load kernel is 3 % faster over a whole run; SERFSIM_TMA=1 selects the TMA pipeline
-    if (const char* e = getenv("SERFSIM_TMA")) use = atoi(e);
-    const u32 need = std::max<u32>(h->max_tile_edges * 4u, 16u);
-    if (use && h->R == 1 && need <= 48u * 1024u) h->stage_col_bytes = (need + 127u) & ~127u;
-  }
-  h->grid = tick_grid_size(h->count, h->stage_col_bytes ? 3 : h->ctas_per_sm);
-  if (getenv("SERFSIM_VERBOSE")) fprintf(stderr, "serfsim: tick kernel = %s (stage_col_bytes %u, grid %d)\n", h->stage_col_bytes ? "tick_kernel_tma" : "tick_kernel", h->stage_col_bytes, h->grid);
+  if (getenv("SERFSIM_VERBOSE")) fprintf(stderr, "serfsim: tick kernel = tick_kernel (grid %d)\n", h->grid);
   h->has_topo = true;
   h->watch_dirty = true;
   return refresh_watchers(h);

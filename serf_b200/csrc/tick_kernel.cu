@@ -19,10 +19,7 @@
 // four neighbour gathers stay inside the node's own 64-byte CSR row; the sends are 32-bit RED.MAX to random peers with
 // an evict_last policy — the inbox planes are the only randomly addressed data and are sized to stay L2-resident.
 // Tiles (256 nodes) nobody delivered to and that hold no pending work are skipped outright in sparse ticks.
-// A TMA variant (tick_kernel_tma) stages whole tiles through cp.async.bulk + mbarrier; the multi-GPU variant stages
-// cross-shard entries in shared memory and stores them into the peer GPU's window over NVLink.
-#include <cstdlib>
-
+// The multi-GPU variant stages cross-shard entries in shared memory and stores them into the peer GPU's window over NVLink.
 #include "tick_kernel.cuh"
 #include "byz.cuh"
 
@@ -31,15 +28,10 @@ namespace sfs {
 namespace {
 
 constexpr int BLOCK = 256;
-#ifndef SFS_MB_R1
-#define SFS_MB_R1 4                         // resident CTAs per SM of the single-slot kernels (64 registers per thread)
-#endif
-#ifndef SFS_MB_R1S
-#define SFS_MB_R1S SFS_MB_R1                // … of the sharded single-slot kernel (its send path needs more registers: A/B in profiles/r2_notes.md)
-#endif
-#ifndef SFS_MB_RN
-#define SFS_MB_RN 2                         // resident CTAs per SM of the multi-slot kernels (128 registers per thread: at 3 CTAs / 80 registers the
-#endif                                      // view loop spills, and local-memory traffic goes through the LSU the kernel is bound by: −7 % per run, profiles/r2_notes.md)
+constexpr int MB_R1 = 4;                    // resident CTAs per SM of the single-slot kernels (64 registers per thread)
+constexpr int MB_R1S = MB_R1;               // … of the sharded single-slot kernel (its send path needs more registers: A/B in profiles/r2_notes.md)
+constexpr int MB_RN = 2;                    // resident CTAs per SM of the multi-slot kernels (128 registers per thread: at 3 CTAs / 80 registers the
+                                            // view loop spills, and local-memory traffic goes through the LSU the kernel is bound by: −7 % per run, profiles/r2_notes.md)
 constexpr u32 TILE_SHIFT = 8;              // one tile = one CTA pass = 256 nodes
 constexpr u32 MAX_TILES_PER_CTA = 1024;
 static_assert((1u << TILE_SHIFT) == BLOCK, "tile = block");
@@ -105,37 +97,6 @@ inline u32 ld_acquire_sys(const u32* ptr) {                 // polled in a loop 
 }
 #endif
 
-#ifndef SERFSIM_EMU
-// ---- TMA (bulk async copy) + mbarrier plumbing: stages a whole 256-node tile into shared memory ----
-__device__ __forceinline__ u32 smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64* bar, u32 count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_arrive_expect_tx(u64* bar, u32 bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(u64* bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(smem_u32(bar)) : "memory"); }
-__device__ __forceinline__ void mbar_wait(u64* bar, u32 parity) {
-  u32 ok;
-  do {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  } while (!ok);
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// global → shared bulk copy (UBLKCP); completion is signalled on `bar` as transaction bytes
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, u32 bytes, u64* bar, u64 pol) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-               :: "r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(pol) : "memory");
-}
-#endif
-
-// Shared-memory image of one tile (single-slot runs): everything the 256 nodes of the tile read this tick.
-constexpr u32 ST_REC = 0, ST_NODE = 8192, ST_INL = 10240, ST_INJ = 11264, ST_INM = 12288, ST_RP = 13312, ST_COL = 14400;
-constexpr u32 RP_BYTES = 1040;             // 260 row offsets (257 needed, rounded to 16 B)
-struct StageView {
-  const Words* rec; const u64* node; const u32* inL; const u32* inJ; const u32* inM; const u32* rowptr; const u32* col;
-  u32 col_base;                            // first CSR element held in `col`
-  bool col_staged;                         // false: the tile's CSR span exceeds the stage; gather from global memory
-};
-
 struct Counters {          // per-thread, reduced once per CTA; rare counters (events, suspects) go straight to the trace row
   u32 packets, edges, changed, pending, kL, kJ, kM, views;
   // single-view kernels (64 registers per thread, on the edge of spilling) keep six of them in three: a thread visits at most
@@ -188,19 +149,10 @@ __device__ __forceinline__ void deliver(const TickParams& p, XStage* xs, u32* pl
     u32 dloc;
     const u32 shard = shard_of(p, dst, dloc);
     const u64 e = ((u64)val1 << 32) | ((u64)(s + p.sv_wshift) << 28) | ((u64)kind << 26) | dloc;   // (a single-view launch numbers its view 0: the entry carries the real one)
-    // warp-aggregated append: the lanes of this call that target the same shard reserve their slots with ONE
-    // shared-memory atomic on the warp's own counter (divergent callers of the same warp may interleave: keep it atomic)
-#ifdef SFS_XSTAGE_MATCH                           // A/B: one shared atomic per distinct shard of the call (match_any + leader + shuffle)
-    const u32 peers = __match_any_sync(__activemask(), shard);
-    const u32 lane = threadIdx.x & 31, wid = threadIdx.x >> 5, leader = __ffs(peers) - 1;
-    u32 base = 0;
-    if (lane == leader) base = atomicAdd(&xs->cnt[wid][shard], (u32)__popc(peers));
-    base = __shfl_sync(peers, base, leader);
-    const u32 pos = base + (u32)__popc(peers & ((1u << lane) - 1u));
-#else                                             // one shared atomic per lane: the hardware serialises the lanes that hit the same counter
+    // append to the warp's own buffer for that shard: one shared-memory atomic per lane on the warp's counter (the hardware
+    // serialises the lanes that hit the same counter; divergent callers of the same warp may interleave: keep it atomic)
     const u32 wid = threadIdx.x >> 5;
     const u32 pos = atomicAdd(&xs->cnt[wid][shard], 1u);
-#endif
     if (pos < xcap(p)) {
       xs->buf[wid * XW_TOTAL + xseg(p, shard) + pos] = e;
     } else {                                   // buffer full: write this one straight through
@@ -298,8 +250,8 @@ constexpr u32 NO_TARGET = 0xffffffffu;
 __device__ __forceinline__ u32 draw16(const u32 (&w)[4], int i) { const u32 x = w[(i >> 1) & 3]; return (i & 1) ? (x >> 16) : (x & 0xffffu); }
 // pick_issue draws the slots and requests the neighbour ids (cand[]: loads in flight), pick_finish drops self slots and packs the targets.
 #define SFS_LD_COL(ptr, pol) __ldg(ptr)     // read-only path WITH L1 allocation: the four picks of a node fall into its two CSR sectors, later picks hit L1 (an evict_first / no-allocate gather was 6 % slower in plateau ticks)
-template <int FMAX, bool STAGED>
-__device__ __forceinline__ void pick_issue(const TickParams& p, const StageView& sv, u32 v, u32 row0, u32 deg, u64 pol_first, u32 (&cand)[FMAX]) {
+template <int FMAX>
+__device__ __forceinline__ void pick_issue(const TickParams& p, u32 v, u32 row0, u32 deg, u64 pol_first, u32 (&cand)[FMAX]) {
   const u32 m = min(p.fanout, deg);
   u32 w[4];
   philox4x32_10(p.tick, v, 0, DOMAIN_GOSSIP, p.seed_lo, p.seed_hi, w);
@@ -313,7 +265,7 @@ __device__ __forceinline__ void pick_issue(const TickParams& p, const StageView&
     for (int i = 0; i < k; ++i) j += (j >= srt[i]) ? 1u : 0u;         // rank → slot: skip the slots already taken
     const bool use = (u32)k < m;
     const u32 e = row0 + (use ? j : 0u);
-    cand[k] = use ? ((STAGED && sv.col_staged) ? sv.col[e - sv.col_base] : SFS_LD_COL(p.col + e, pol_first)) : v;
+    cand[k] = use ? SFS_LD_COL(p.col + e, pol_first) : v;
     // insert j into the ascending list (only if used): bubble it down from position k
     u32 x = use ? j : NO_TARGET;
 #pragma unroll
@@ -390,9 +342,7 @@ __device__ __forceinline__ u32 sleeping_deadline(const Pre& x, bool due) { retur
 // scan) raise the register demand of the path every node takes and make it spill.  They are called on COPIES of the view and
 // the node's scalars: a variable whose address is passed to a call lives in local memory for its whole lifetime, and the
 // hot path's record must stay in registers (measured: 4.6 extra L2 sectors per node and +25 % per plateau tick otherwise).
-#if defined(SFS_COLD_INLINE)
-#define SFS_COLD __forceinline__               // A/B: everything inline again
-#elif defined(SERFSIM_EMU)
+#ifdef SERFSIM_EMU
 #define SFS_COLD __attribute__((noinline))
 #else
 #define SFS_COLD __noinline__
@@ -469,11 +419,9 @@ __device__ SFS_COLD bool cold_can_confirm(u32 k, u32 mask, u32 v) {
 // A view whose only business is a running suspicion timer does not: its deadline goes to `mind` (the caller registers the
 // minimum in tile_due) and the view sleeps until its tile comes due.  `due`: this tile's earliest deadline has been reached —
 // every node of it that carries a timer (busy bit 3) visits all its views.
-template <bool TRACE, int FMAX, bool SHARDED, bool R1, bool STAGED>
-__device__ __forceinline__ bool process_node(const TickParams& p, const StageView& sv, XStage* xs, const u32 vl, const Pre& pre, const bool kL, const bool kJ, const bool kM, const bool mark, const bool saturated,
+template <bool TRACE, int FMAX, bool SHARDED, bool R1>
+__device__ __forceinline__ bool process_node(const TickParams& p, XStage* xs, const u32 vl, const Pre& pre, const bool kL, const bool kJ, const bool kM, const bool mark, const bool saturated,
                                              const bool due, const u64 pol_first, const u64 pol_last, Counters& c, u32& mind, int& dsusp, const Ahead<FMAX>& ah, u32& first_view, const u32 sv_views = 0xffffffffu) {
-  static_assert(!STAGED || R1, "the staged path is the single-slot path");
-  const u32 lt = threadIdx.x;              // index inside the staged tile
   const u32 v = p.first + vl;
   const u32 t = p.tick;
   const u32 limit = p.rules.limit;
@@ -484,40 +432,32 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
   // needs is requested up front, independent loads in flight together.  Otherwise most nodes are idle: read only
   // the busy byte and the inbox words, and fetch the 8-byte node word and the 32-byte record just for the nodes
   // that have something to do.  Multi-slot runs fetch the records of the views that have something to do. ----
-  const bool upfront = R1 && (saturated || TRACE || STAGED);
+  const bool upfront = R1 && (saturated || TRACE);
   u64 ns = 0;
   u32 row0 = 0, row1 = 0;
   Words cur;
   auto load_node = [&]() {
-    ns = STAGED ? sv.node[lt] : ld_u64_stream(p.node_state + vl, pol_first);
-    if (STAGED) { row0 = sv.rowptr[lt]; row1 = sv.rowptr[lt + 1]; }
-    else if (p.udeg) { row0 = vl * p.udeg; row1 = row0 + p.udeg; }     // uniform out-degree: the row offsets are arithmetic
+    ns = ld_u64_stream(p.node_state + vl, pol_first);
+    if (p.udeg) { row0 = vl * p.udeg; row1 = row0 + p.udeg; }     // uniform out-degree: the row offsets are arithmetic
     else { row0 = __ldg(p.row_ptr + vl); row1 = __ldg(p.row_ptr + vl + 1); }
   };
   auto load_rec0 = [&]() {
-    if (STAGED) {
-      const uint4 a = reinterpret_cast<const uint4*>(sv.rec + lt)[0], b = reinterpret_cast<const uint4*>(sv.rec + lt)[1];
-      cur.w[0] = a.x; cur.w[1] = a.y; cur.w[2] = a.z; cur.w[3] = a.w; cur.w[4] = b.x; cur.w[5] = b.y; cur.w[6] = b.z; cur.w[7] = b.w;
-    } else {
-      cur = ld_rec256(p.rec + 2 * (size_t)vl, pol_first);
-    }
+    cur = ld_rec256(p.rec + 2 * (size_t)vl, pol_first);
     merge_q(cur, pre.qw);                                  // the record image everything below works on is record | budgets
   };
   if (upfront) { load_node(); load_rec0(); }
   const u32 busy = pre.busy;
   u32 mL = pre.mL, mJ = pre.mJ, mM = pre.mM;
-  if (STAGED) { mL = kL ? sv.inL[lt] : 0u; mJ = kJ ? sv.inJ[lt] : 0u; mM = kM ? sv.inM[lt] : 0u; }
 
   // ---- idle exit: nothing received (any slot), nothing queued, no host operation, no probe duty, no timer due ----
   u32 nd = pre.nd;                                       // the node's own earliest deadline: matters in due tiles, for nodes that run timers
   if (R1 && due && (busy & 8u)) nd = p.node_due[vl];
   const u32 sleeping = (due && (busy & 8u)) ? nd : NO_DEADLINE;
   const bool timers_due = sleeping <= p.tick;
-  if (!TRACE && !STAGED && !((busy & 7u) != 0 || pre.any != 0 || p.reap_now != 0 || timers_due)) { mind = min(mind, sleeping); if (due && (busy & 8u)) SFS_PROBE(20); return false; }
-  if (STAGED && !TRACE && !((busy & 7u) || (mL | mJ | mM) || p.reap_now || timers_due)) { mind = min(mind, sleeping); return false; }
+  if (!TRACE && !((busy & 7u) != 0 || pre.any != 0 || p.reap_now != 0 || timers_due)) { mind = min(mind, sleeping); if (due && (busy & 8u)) SFS_PROBE(20); return false; }
   // (the watcher mask — subjects this node can probe, it has them as neighbours — is re-read where a watcher needs it: a handful of nodes)
 #define SFS_WMASK() ((busy & 4u) ? ((u32)p.watch[vl] >> p.sv_wshift) : 0u)   /* sv_wshift: the view a single-view launch works on (0 in every other launch) */
-  const bool ahead = !R1 && !STAGED && ah.valid;       // node word, peers' ids and the record of view pre.keep were requested a tile ago
+  const bool ahead = !R1 && ah.valid;                  // node word, peers' ids and the record of view pre.keep were requested a tile ago
   if (ahead) { ns = ah.ns; row0 = vl * p.udeg; row1 = row0 + p.udeg; }
   else if (!upfront) { load_node(); if (R1) load_rec0(); }
 
@@ -537,12 +477,7 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
   bool have_probe = false;
   u32 ptarget = 0;
   if (up_s && (busy & 4u) && p.probe_every && p.down_mask && ((t + v) % p.probe_every) == 0 && deg) {
-    ptarget = (STAGED && sv.col_staged) ? 0u : cold_probe_target(p, v, row0, deg);
-    if (STAGED && sv.col_staged) {
-      u32 w[4];
-      philox4x32_10(t, v, 0, DOMAIN_PROBE, p.seed_lo, p.seed_hi, w);
-      ptarget = sv.col[row0 + (((w[0] & 0xffffu) * deg) >> 16) - sv.col_base];
-    }
+    ptarget = cold_probe_target(p, v, row0, deg);
     have_probe = true;
   }
 
@@ -560,7 +495,8 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
   u32 todo = visit_all ? all_views : ((pre.mailmask | pre.qmask | (p.probe_every ? (SFS_WMASK() & p.down_mask) : 0u)) & all_views);
   if (!R1) SFS_COUNT(5, R - (u32)__popc(todo));             // views left asleep by a visited node
 
-  // multi-slot runs: the record and inbox words of the next view to visit are requested while the current one is processed
+  // multi-slot runs: the record and inbox words of the next view to visit are requested once the current one is stored
+  // (requesting them while it is processed keeps 12 more registers live and was measured slower)
   Words nxt = {};
   u32 nL = 0, nJ = 0, nM = 0, nq = 0;
   auto load_view = [&](u32 s2, Words& w, u32& q, u32& iL, u32& iJ, u32& iM) {
@@ -573,9 +509,6 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
     iJ = kJ ? ld_u32_stream(p.inbox_rd + (size_t)(KIND_JOIN * R + s2) * nl + vl, pol_first) : 0;
     iM = kM ? ld_u32_stream(p.inbox_rd + (size_t)(KIND_ML * R + s2) * nl + vl, pol_first) : 0;
   };
-#ifndef SFS_VIEW_PREFETCH
-#define SFS_VIEW_PREFETCH 0                  // 1: the next view's record is requested while the current one is processed (12 more live registers; measured slower)
-#endif
   u32 s = R;
   if (R1) { s = 0; todo = 0; }
   else if (todo) {
@@ -590,7 +523,7 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
   while (s < R) {
     const size_t idx = (size_t)s * nl + vl;
     u32 s_next = R;
-    if (!R1 && todo) { s_next = (u32)__ffs((int)todo) - 1u; todo &= todo - 1u; if (SFS_VIEW_PREFETCH) load_view(s_next, nxt, nq, nL, nJ, nM); }
+    if (!R1 && todo) { s_next = (u32)__ffs((int)todo) - 1u; todo &= todo - 1u; }
     if (mL) st_u32_stream(p.inbox_rd + (size_t)(KIND_LEAVE * R + s) * nl + vl, 0u, pol_first);   // consume: clear for reuse in two ticks
     if (mJ) st_u32_stream(p.inbox_rd + (size_t)(KIND_JOIN * R + s) * nl + vl, 0u, pol_first);
     if (mM) st_u32_stream(p.inbox_rd + (size_t)(KIND_ML * R + s) * nl + vl, 0u, pol_first);
@@ -634,7 +567,7 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
           if (ahead) nt = pick_finish<FMAX>(v, ah.cand, tg);
           else {
             u32 cand[FMAX];
-            pick_issue<FMAX, STAGED>(p, sv, v, row0, deg, pol_first, cand);
+            pick_issue<FMAX>(p, v, row0, deg, pol_first, cand);
             nt = pick_finish<FMAX>(v, cand, tg);
           }
           have_targets = true;
@@ -682,7 +615,7 @@ __device__ __forceinline__ bool process_node(const TickParams& p, const StageVie
     if (TRACE) c.hash += rec_hash((u64)s * p.n_global + v, make_uint4(cur.w[0], cur.w[1], cur.w[2], cur.w[3]), make_uint4(cur.w[4], cur.w[5], cur.w[6], cur.w[7]));
     if (r.inc >= INC_LIMIT) *p.overflow = 1;
     if (!R1) {
-      if (!SFS_VIEW_PREFETCH && s_next < R) load_view(s_next, nxt, nq, nL, nJ, nM);
+      if (s_next < R) load_view(s_next, nxt, nq, nL, nJ, nM);
       cur = nxt; merge_q(cur, nq); mL = nL; mJ = nJ; mM = nM;
     }
     s = s_next;
@@ -978,7 +911,7 @@ __global__ void __launch_bounds__(BLOCK, MB) tick_kernel(const __grid_constant__
           }
           u32 mind = NO_DEADLINE, fv_unused = 0;
           int dsusp = 0;
-          const bool pend = process_node<TRACE, FMAX, SHARDED, R1, false>(p, StageView{}, xs, vl, pre, kL, kJ, kM, mark, false, (hot_s[ti] & 2u) != 0, pol_first, pol_last, c, mind, dsusp, Ahead<FMAX>{}, fv_unused, sv_views);
+          const bool pend = process_node<TRACE, FMAX, SHARDED, R1>(p, xs, vl, pre, kL, kJ, kM, mark, false, (hot_s[ti] & 2u) != 0, pol_first, pol_last, c, mind, dsusp, Ahead<FMAX>{}, fv_unused, sv_views);
           if (mark && pend) pend_s[g] = 1;
           if (mind != NO_DEADLINE) atomicMin(p.tile_due + tile0 + ti, mind);      // the list mixes tiles: per-lane registration (few active nodes)
           if (dsusp) atomicAdd(&dsusp_s, dsusp);
@@ -1005,7 +938,7 @@ __global__ void __launch_bounds__(BLOCK, MB) tick_kernel(const __grid_constant__
     if (!R1 && ahead_on && vn < p.n_local) {
       a.ns = ld_u64_stream(p.node_state + vn, pol_first);
       a.rec = ld_rec256(p.rec + 2 * ((size_t)keep * p.stride + vn), pol_first);
-      pick_issue<FMAX, false>(p, StageView{}, p.first + vn, vn * p.udeg, p.udeg, pol_first, a.cand);
+      pick_issue<FMAX>(p, p.first + vn, vn * p.udeg, p.udeg, pol_first, a.cand);
       a.valid = 1;
       SFS_PROBE(19);
     }
@@ -1026,7 +959,7 @@ __global__ void __launch_bounds__(BLOCK, MB) tick_kernel(const __grid_constant__
     bool pend = false;
     u32 mind = NO_DEADLINE;
     int dsusp = 0;
-    if (vl < p.n_local) pend = process_node<TRACE, FMAX, SHARDED, R1, false>(p, StageView{}, xs, vl, pre, kL, kJ, kM, mark, saturated, (hot_s[i] & 2u) != 0, pol_first, pol_last, c, mind, dsusp, ah, first_view, sv_views);
+    if (vl < p.n_local) pend = process_node<TRACE, FMAX, SHARDED, R1>(p, xs, vl, pre, kL, kJ, kM, mark, saturated, (hot_s[i] & 2u) != 0, pol_first, pol_last, c, mind, dsusp, ah, first_view, sv_views);
     if (mark && __any_sync(0xffffffffu, pend) && lane == 0) p.hot_wr[tile0 + i] = 1;
     note_timers(p, tile0 + i, mind, dsusp, &dsusp_s);
     if (SHARDED) wrote_remote |= flush_xwarp(p, xs, false, resv, rlen);
@@ -1040,117 +973,6 @@ __global__ void __launch_bounds__(BLOCK, MB) tick_kernel(const __grid_constant__
   __syncthreads();
   finish_tick<TRACE, R1>(p, c, red, dsusp_s);
 }
-
-#ifndef SERFSIM_EMU   // the TMA pipeline is device-only (bulk copies, mbarriers); the host build of tests/emu uses the direct-load kernel
-// The same tick for single-slot runs with the whole working set of a tile staged through TMA: one elected
-// thread bulk-copies the tile's records (8 KB), node words (2 KB), live inbox planes (1 KB each), row offsets
-// (1 KB) and CSR span (the tile's neighbour lists, 16 KB at out-degree 16) into shared memory, one tile ahead
-// of the 256 consumers (2 stages, mbarrier transaction counts).  The node logic then runs out of shared memory;
-// only the RED.MAX sends, the record write-back and the inbox clears touch global memory from the LSU.
-template <bool TRACE, int FMAX, bool SHARDED, bool BARSYNC>
-__global__ void __launch_bounds__(BLOCK, 3) tick_kernel_tma(const __grid_constant__ TickParams p) {
-  extern __shared__ __align__(128) unsigned char stage_mem[];
-  __shared__ u8 hot_s[MAX_TILES_PER_CTA];
-  __shared__ u16 hot_list[MAX_TILES_PER_CTA];
-  __shared__ u32 n_hot_s;
-  __shared__ u64 red[8][BLOCK / 32];
-  __shared__ __align__(8) u64 full_bar[2], empty_bar[2];
-  __shared__ u32 col_base_s[2], col_ok_s[2];
-  __shared__ int dsusp_s;
-  if (gate_closed(p.gate, blockIdx.x == 0 && threadIdx.x == 0)) return;
-  if (tick_is_idle(p.sched, p.tick, p.ev_begin, p.ev_end)) { write_idle_row<TRACE>(p); return; }
-  Counters c = {};
-  const bool kL = p.kinds_prev[KIND_LEAVE] != 0, kJ = p.kinds_prev[KIND_JOIN] != 0, kM = p.kinds_prev[KIND_ML] != 0;
-  const u64 pol_first = policy_evict_first(), pol_last = policy_evict_last();
-  const int lane = threadIdx.x & 31;
-
-  const u32 prev_msgs = p.kinds_prev[KIND_LEAVE] + p.kinds_prev[KIND_JOIN] + p.kinds_prev[KIND_ML];
-  const bool dense_now = prev_msgs >= (p.n_tiles >> 1) + 1;
-  const bool all_hot = p.force_all || p.kinds_prev[3] != 0;
-  const bool mark = !dense_now;
-  if (dense_now && blockIdx.x == 0 && threadIdx.x == 0) p.kinds_cur[3] = 1;
-
-  const u32 tile0 = blockIdx.x * p.tiles_per_cta;
-  const u32 ntile = tile0 < p.n_tiles ? min(p.tiles_per_cta, p.n_tiles - tile0) : 0;
-  scan_tiles(p, hot_s, tile0, ntile, all_hot);
-  if (threadIdx.x == 0) {
-    dsusp_s = 0;
-    mbar_init(&full_bar[0], 1); mbar_init(&full_bar[1], 1);
-    mbar_init(&empty_bar[0], BLOCK / 32); mbar_init(&empty_bar[1], BLOCK / 32);     // one arrival per consumer warp
-    fence_proxy_async();
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    u32 n = 0;
-    for (u32 i = 0; i < ntile; ++i) if (hot_s[i]) hot_list[n++] = (u16)i;
-    n_hot_s = n;
-  }
-  __syncthreads();
-  const u32 n_hot = n_hot_s;
-  const u32 stage_bytes = ST_COL + p.stage_col_bytes;
-
-  // producer: bulk-copy tile `j` of the hot list into stage j&1
-  auto issue = [&](u32 j) {
-    const u32 st = j & 1;
-    unsigned char* base = stage_mem + (size_t)st * stage_bytes;
-    const u32 tile = tile0 + hot_list[j];
-    const u32 v0 = tile << TILE_SHIFT;
-    const u32 e0 = __ldg(p.row_ptr + v0) & ~3u;
-    const u32 e1 = (__ldg(p.row_ptr + min(v0 + BLOCK, p.n_local)) + 3u) & ~3u;
-    const u32 col_bytes = (e1 - e0) * 4u;
-    const bool col_ok = col_bytes != 0 && col_bytes <= p.stage_col_bytes;
-    col_base_s[st] = e0; col_ok_s[st] = col_ok ? 1u : 0u;
-    const u32 tx = 8192u + 2048u + RP_BYTES + (kL ? 1024u : 0u) + (kJ ? 1024u : 0u) + (kM ? 1024u : 0u) + (col_ok ? col_bytes : 0u);
-    fence_proxy_async();                                   // earlier generic reads of this stage precede the async writes
-    mbar_arrive_expect_tx(&full_bar[st], tx);
-    bulk_g2s(base + ST_REC, p.rec + 2 * (size_t)v0, 8192u, &full_bar[st], pol_first);
-    bulk_g2s(base + ST_NODE, p.node_state + v0, 2048u, &full_bar[st], pol_first);
-    bulk_g2s(base + ST_RP, p.row_ptr + v0, RP_BYTES, &full_bar[st], pol_first);
-    if (kL) bulk_g2s(base + ST_INL, p.inbox_rd + (size_t)KIND_LEAVE * p.stride + v0, 1024u, &full_bar[st], pol_first);
-    if (kJ) bulk_g2s(base + ST_INJ, p.inbox_rd + (size_t)KIND_JOIN * p.stride + v0, 1024u, &full_bar[st], pol_first);
-    if (kM) bulk_g2s(base + ST_INM, p.inbox_rd + (size_t)KIND_ML * p.stride + v0, 1024u, &full_bar[st], pol_first);
-    if (col_ok) bulk_g2s(base + ST_COL, p.col + e0, col_bytes, &full_bar[st], pol_first);
-  };
-
-  // No CTA-wide barrier in the loop: a warp that finishes a tile arrives on the stage's `empty` barrier and
-  // moves on; only the producer (thread 0) waits for all eight warps to release a stage before refilling it.
-  if (threadIdx.x == 0 && n_hot) issue(0);
-  for (u32 j = 0; j < n_hot; ++j) {
-    if (threadIdx.x == 0 && j + 1 < n_hot) {
-      if (!BARSYNC && j >= 1) mbar_wait(&empty_bar[(j + 1) & 1], ((j - 1) >> 1) & 1);   // tile j-1 (same stage) fully consumed
-      issue(j + 1);
-    }
-    const u32 st = j & 1;
-    mbar_wait(&full_bar[st], (j >> 1) & 1);
-    unsigned char* base = stage_mem + (size_t)st * stage_bytes;
-    StageView sv;
-    sv.rec = reinterpret_cast<const Words*>(base + ST_REC); sv.node = reinterpret_cast<const u64*>(base + ST_NODE);
-    sv.inL = reinterpret_cast<const u32*>(base + ST_INL); sv.inJ = reinterpret_cast<const u32*>(base + ST_INJ); sv.inM = reinterpret_cast<const u32*>(base + ST_INM);
-    sv.rowptr = reinterpret_cast<const u32*>(base + ST_RP); sv.col = reinterpret_cast<const u32*>(base + ST_COL);
-    sv.col_base = col_base_s[st]; sv.col_staged = col_ok_s[st] != 0;
-    const u32 ti = hot_list[j];
-    const u32 vl = ((tile0 + ti) << TILE_SHIFT) + threadIdx.x;
-    bool pend = false;
-    u32 mind = NO_DEADLINE;
-    int dsusp = 0;
-    if (vl < p.n_local) {
-      Pre pre = {};
-      pre.busy = p.busy[vl];
-      pre.qw = p.qword[vl];          // 4 B per node, read directly (not worth a sixth bulk copy per stage)
-      pre.nd = NO_DEADLINE;
-      u32 fv_unused = 0;
-      pend = process_node<TRACE, FMAX, false, true, true>(p, sv, nullptr, vl, pre, kL, kJ, kM, mark, true, (hot_s[ti] & 2u) != 0, pol_first, pol_last, c, mind, dsusp, Ahead<FMAX>{}, fv_unused);
-    }
-    if (mark && __any_sync(0xffffffffu, pend) && lane == 0) p.hot_wr[tile0 + ti] = 1;
-    note_timers(p, tile0 + ti, mind, dsusp, &dsusp_s);
-    if (BARSYNC) __syncthreads();
-    else { __syncwarp(); if (lane == 0) mbar_arrive(&empty_bar[st]); }     // this warp is done reading stage `st`
-  }
-
-  __syncthreads();
-  finish_tick<TRACE, true>(p, c, red, dsusp_s);
-}
-#endif
 
 // Anti-entropy round — memberlist push-pull + SerfDelegate::merge_remote_state (serf/delegate.rs:386-554; "next"
 // row 1 of SURVEY §8f).  Runs after the tick kernel every push_pull_interval ticks on a SNAPSHOT of the end-of-tick
@@ -1519,9 +1341,9 @@ __global__ void __launch_bounds__(BLOCK) summary_kernel(const uint4* rec, const 
 
 }  // namespace
 
-int tick_ctas_per_sm_r1() { return SFS_MB_R1; }
-int tick_ctas_per_sm_r1s() { return SFS_MB_R1S; }
-int tick_ctas_per_sm_rn() { return SFS_MB_RN; }
+int tick_ctas_per_sm_r1() { return MB_R1; }
+int tick_ctas_per_sm_r1s() { return MB_R1S; }
+int tick_ctas_per_sm_rn() { return MB_RN; }
 int tick_grid_size(u32 n_local, int ctas_per_sm) {
   static int sms = 0;
   if (!sms) {
@@ -1531,45 +1353,18 @@ int tick_grid_size(u32 n_local, int ctas_per_sm) {
     if (sms <= 0) sms = 148;
   }
   const u32 tiles = (n_local + BLOCK - 1) / BLOCK;
-  static int mul = 0;
-  if (!mul) { const char* e = getenv("SERFSIM_GRIDMUL"); mul = e ? atoi(e) : 2; if (mul < 1) mul = 2; }
-  u32 grid = (u32)sms * (u32)ctas_per_sm * (u32)mul;    // persistent: SM count × resident CTAs × 2 (two waves for balance)
+  u32 grid = (u32)sms * (u32)ctas_per_sm * 2u;          // persistent: SM count × resident CTAs × 2 (two waves for balance)
   if (tiles < grid) grid = tiles ? tiles : 1;
   while ((tiles + grid - 1) / grid > MAX_TILES_PER_CTA) grid += (u32)sms * (u32)ctas_per_sm;
   return (int)grid;
 }
 
-#ifndef SERFSIM_EMU
-template <bool TRACE, int FMAX, bool SHARDED>
-static void launch_tick_tma(const TickParams& p, int grid, cudaStream_t st) {
-  const size_t smem = 2 * (size_t)(ST_COL + p.stage_col_bytes);
-  static bool configured = false;
-  static int barsync = 0;
-  if (!configured) {
-    cudaFuncSetAttribute(tick_kernel_tma<TRACE, FMAX, SHARDED, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(tick_kernel_tma<TRACE, FMAX, SHARDED, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (const char* e = getenv("SERFSIM_TMA_SYNC")) barsync = atoi(e);
-    configured = true;
-  }
-  if (barsync) SFS_LAUNCH(grid, BLOCK, smem, st, tick_kernel_tma<TRACE, FMAX, SHARDED, true>)(p);
-  else SFS_LAUNCH(grid, BLOCK, smem, st, tick_kernel_tma<TRACE, FMAX, SHARDED, false>)(p);
-}
-#endif
-
 template <bool TRACE, int FMAX>
 static void launch_tick_v(const TickParams& p, int grid, cudaStream_t st) {
   const bool sharded = p.world > 1, r1 = p.R == 1;
-#ifndef SERFSIM_EMU
-  if (r1 && p.stage_col_bytes && !sharded) { // single-slot, single-GPU run whose tiles fit a shared-memory stage: TMA pipeline
-    launch_tick_tma<TRACE, FMAX, false>(p, grid, st);
-    return;
-  }
-#endif
-  static int mb5 = -1;
-  if (mb5 < 0) { const char* e = getenv("SERFSIM_MINB"); mb5 = (e && atoi(e) == 5) ? 1 : 0; }
-  if (sharded) { if (r1) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, true, true, SFS_MB_R1S>)(p); else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, true, false, SFS_MB_RN>)(p); }
-  else if (r1) { if (mb5) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, false, true, 5>)(p); else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, false, true, SFS_MB_R1>)(p); }
-  else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, false, false, SFS_MB_RN>)(p);
+  if (sharded) { if (r1) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, true, true, MB_R1S>)(p); else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, true, false, MB_RN>)(p); }
+  else if (r1) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, false, true, MB_R1>)(p);
+  else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<TRACE, FMAX, false, false, MB_RN>)(p);
 }
 void launch_tick(const TickParams& p, bool trace, int grid, cudaStream_t st) {
   const bool small = p.fanout <= 4;          // the common fan-outs (3, 4) get the 4-wide target array
@@ -1580,11 +1375,11 @@ void launch_tick(const TickParams& p, bool trace, int grid, cudaStream_t st) {
 void launch_tick_single_view(const TickParams& p, int grid, cudaStream_t st) {
   const bool sharded = p.world > 1;
   if (p.fanout <= 4) {
-    if (sharded) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 4, true, true, SFS_MB_R1S>)(p);
-    else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 4, false, true, SFS_MB_R1>)(p);
+    if (sharded) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 4, true, true, MB_R1S>)(p);
+    else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 4, false, true, MB_R1>)(p);
   } else {
-    if (sharded) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 8, true, true, SFS_MB_R1S>)(p);
-    else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 8, false, true, SFS_MB_R1>)(p);
+    if (sharded) SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 8, true, true, MB_R1S>)(p);
+    else SFS_LAUNCH(grid, BLOCK, 0, st, tick_kernel<false, 8, false, true, MB_R1>)(p);
   }
 }
 void launch_fill_idle_rows(u64* rows, u64* grow_rows, u32 n, const u32* sched, bool trace, cudaStream_t st) {

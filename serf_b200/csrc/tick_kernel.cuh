@@ -91,8 +91,8 @@ struct TickParams {
   u32* overflow;              // set when a Lamport time / incarnation nears the device width
   u8* hot_rd;                 // [n_tiles] tile flags set during the previous tick (deliveries, pending work, host ops)
   u8* hot_wr;                 // [n_tiles] tile flags for the next tick
-  u32 stage_col_bytes, reap_now, pad2, pad3;         // reap_now: this tick the reaper runs (every view is visited)
-  u32 tombstone_ticks, reconnect_ticks, intent_ticks, pad4;             // > 0: single-slot TMA pipeline with this many bytes of CSR per stage
+  u32 pad1, reap_now, pad2, pad3;         // reap_now: this tick the reaper runs (every view is visited); pad1 keeps the offsets of the members below
+  u32 tombstone_ticks, reconnect_ticks, intent_ticks, pad4;
   u32 n_tiles, tiles_per_cta, force_all, stride;   // stride: plane stride in nodes = n_local rounded up to a whole tile
   // cross-shard exchange (world_size > 1): every rank owns one receive window per peer (mapped into the
   // peers with CUDA IPC); the tick kernel stages cross-shard entries per destination shard in shared memory

@@ -76,6 +76,10 @@ def test_config1_random_graph_100k(seed):
     assert (g.member_status(0)[1:] != MemberStatus.LEFT).sum() <= 3 and ticks < 100     # a random digraph may strand a node or two
 
 
+def test_random_graph_fanout4_ragged_tail():
+    run_both(scenarios.random_graph_leave(60_001, 12, 4, seed=5))          # single slot, last tile partly filled
+
+
 def test_random_graph_multi_slot_fanout4():
     run_both(scenarios.random_graph_leave(60_000, 16, 4, seed=5, slots=4))
 
@@ -85,6 +89,12 @@ def test_failure_detection_random_graph():
     g, o, ticks = run_both(sc, suspicion_mult=2, suspicion_max_timeout_mult=2, probe_interval_ticks=2)
     st = g.member_status(0)
     assert (np.delete(st, 5) == MemberStatus.FAILED).all()
+
+
+def test_failure_detection_single_subject():
+    sc = scenarios.random_graph_fail(20_000, 16, 3, seed=2)
+    sc.slots, sc.subjects, sc.ops = 1, sc.subjects[:1], [op for op in sc.ops if op[2] == int(sc.subjects[0])]
+    run_both(sc, suspicion_mult=2, suspicion_max_timeout_mult=2, probe_interval_ticks=2)
 
 
 def test_failure_detection_lifeguard_confirmations():
@@ -113,6 +123,13 @@ def test_push_pull_anti_entropy(pp):
 @pytest.mark.parametrize("seed", range(40))
 def test_fuzz(seed):
     sc = scenarios.fuzz(seed)
+    sc.max_ticks = 1500
+    run_both(sc)
+
+
+@pytest.mark.parametrize("seed", range(12))
+def test_fuzz_single_slot(seed):
+    sc = scenarios.fuzz(seed, slots=1)
     sc.max_ticks = 1500
     run_both(sc)
 

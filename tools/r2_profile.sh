@@ -1,5 +1,5 @@
 #!/bin/bash
-# Second GPU call of round 2 (after tools/r2_verify.sh decided which kernel variant stays): the ncu evidence bench.py's
+# Second GPU call of round 2 (after the first decided which kernel variant stays): the ncu evidence bench.py's
 # roofline object refers to.  One GPU; ncu replays kernels, so nothing printed by these commands is a bench value.
 #   gpurun --timeout 1800 -- 'bash tools/r2_profile.sh'
 # then here:  python tools/ncu_summary.py gpurun_out/r2_tick13.ncu-rep > profiles/r2_ncu_tick13.txt   (etc.)

@@ -41,10 +41,13 @@ if __name__ == "__main__":
         print(f"{len(fp)} kernels → {a.write}")
     if a.check:
         ref = json.load(open(a.check))
-        changed = sorted(k for k in ref if fp.get(k) != ref[k])
+        changed = sorted(k for k in ref if k in fp and fp[k] != ref[k])
+        removed = sorted(k for k in ref if k not in fp)
         new = sorted(k for k in fp if k not in ref)
-        print(f"{len(ref) - len(changed)} of {len(ref)} recorded kernels unchanged")
+        print(f"{len(ref) - len(changed) - len(removed)} of {len(ref)} recorded kernels unchanged")
         for k in changed:
             print("  changed:", k)
+        for k in removed:
+            print("  removed:", k)
         for k in new:
             print("  new:    ", k)
